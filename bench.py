@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- fwd+bwd views/sec of the surfel-rasterizer hot path on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -73,7 +73,13 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra configurations (C2, C4, strong point, sustained)")
     ap.add_argument("--streams", type=int, default=1, help="ignored (the views of a step share one launch set)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (images, aux maps, radii, parameter gradients) "
+                         "as DIR/<name>.npy, float32, at most 64 MB in all")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the b200 path only")
+    return args
 
 
 class ClockSampler:
@@ -166,6 +172,24 @@ def timed_steps(step_fn, steps, warmup, flush, world, dev):
     return ms, spread
 
 
+def dump_outputs(out_dir, arrays, budget=64 * 10**6):
+    """Writes each tensor as float32 ``out_dir/<name>.npy``.  Smaller tensors are written whole; one larger than
+    an equal share of the budget still left is replaced by a fixed, seeded sample of its flattened elements
+    (in index order), so that two builds given the same arguments write comparable files."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    left = budget - 256 * len(items)                     # room for the .npy headers
+    for i, (name, t) in enumerate(items):
+        a = t.detach().float().cpu().numpy()
+        share = left // (len(items) - i) // 4
+        if a.size > share:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        left -= 4 * a.size
+
+
 def cpu_baseline(P, size, budget_s=10.0, max_views=8):
     """Oracle port on the host cores: fwd+bwd views of the same workload until ~budget_s of CPU work."""
     from lara_b200 import scene as S
@@ -215,7 +239,9 @@ def make_batched_step(wl, grads, all_reduce=True, coll_events=None):
 
     def step():
         grads.zero_()
-        sharded.render_views(wl.params, wl.sets, None, grads=grads, view_ids=wl.ids, cams=packed, upstream_stacked=G)
+        # (color, allmap, radii) per view of the latest step, for --dump-outputs
+        step.views, _ = sharded.render_views(wl.params, wl.sets, None, grads=grads, view_ids=wl.ids, cams=packed,
+                                             upstream_stacked=G)
         if all_reduce:
             if coll_events is not None:
                 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -440,6 +466,11 @@ def main():
         sampler.start()
     ms, spread = timed_steps(step, args.steps, 0, flush, world, dev)
     value = total_views * args.steps / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        outs = {"color": torch.stack([c for c, _, _ in step.views]), "allmap": torch.stack([a for _, a, _ in step.views]),
+                "radii": torch.stack([r for _, _, r in step.views])}
+        outs.update({"grad_" + k: v for k, v in grads.views.items()})
+        dump_outputs(args.dump_outputs, outs)
     collective_us = None
     rank_compute_ms = None
     if coll:

@@ -1,79 +1,31 @@
 """Decoder epilogue (next-row, SURVEY 8f rank 4): MLP output -> contiguous Gaussian-parameter tensors.
 
-* CPU, only where /root/reference exists: the torch restatement is pinned bit-exactly against the reference's own
-  ``Decoder.forward_coarse`` + ``Network.get_offseted_pt`` (lightning/network.py), imported with stub modules for
-  the packages this image lacks (timm, pytorch_lightning) and an identity MLP.
+* CPU: the torch restatement is pinned bit-exactly against what the reference's own ``Decoder.forward_coarse`` +
+  ``Network.get_offseted_pt`` (lightning/network.py) compute with an identity MLP (tests/golden/reference, made by
+  tests/golden/make_reference_golden.py).
 * GPU: the fused kernel vs the restatement -- forward values bit-exact except the sigmoid path (<= 2 ulp), backward
   to 1e-6."""
-import os
-import sys
-import types
-
 import pytest
 import torch
 
-from helpers import rel_err
+from helpers import Reference, rel_err
 
-REF_ROOT = "/root/reference"
-
-
-def _import_reference_network():
-    stubs = {}
-
-    def stub(name, **attrs):
-        m = types.ModuleType(name)
-        for k, v in attrs.items():
-            setattr(m, k, v)
-        stubs[name] = m
-        return m
-    stub("timm")
-    stub("pytorch_lightning", LightningModule=torch.nn.Module)
-    tv = stub("torchvision")
-    tv.transforms = stub("torchvision.transforms")
-    saved = {k: sys.modules.get(k) for k in stubs}
-    sys.modules.update({k: v for k, v in stubs.items() if k not in sys.modules or k in ("timm", "pytorch_lightning")})
-    sys.path.insert(0, REF_ROOT)
-    try:
-        import importlib
-        for k in [k for k in sys.modules if k == "lightning" or k.startswith("lightning.")]:
-            del sys.modules[k]
-        net = importlib.import_module("lightning.network")
-    finally:
-        sys.path.remove(REF_ROOT)
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
-            else:
-                sys.modules[k] = v
-        for k in [k for k in sys.modules if k == "lightning" or k.startswith("lightning.") or k == "tools" or k.startswith("tools.")]:
-            del sys.modules[k]
-    return net
+def decoder_inputs():
+    """MLP output features (identity MLP), group centres, K, sh_dim, opacity and scaling shifts."""
+    B, N, K, sh_dim = 2, 27, 2, 12
+    g = torch.Generator().manual_seed(0)
+    feats = torch.randn((B, N, K * (10 + sh_dim)), generator=g)
+    centers_grid = torch.rand((1, N, 3), generator=g) - 0.5
+    return feats, centers_grid, K, sh_dim, -2.1792, -4.2
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF_ROOT, "lightning")), reason="/root/reference not present (GPU box)")
 def test_decoder_restatement_matches_reference_on_cpu():
     from oracle.torch_restatements import decoder_layout_torch
-    try:
-        net = _import_reference_network()
-    except Exception as ex:           # a package the reference imports at module level is missing here
-        pytest.skip(f"reference network.py not importable in this image: {ex!r}")
-    B, N, K, sh_dim = 2, 27, 2, 12
-    C = 10 + sh_dim
-    g = torch.Generator().manual_seed(0)
-    feats = torch.randn((B, N, K * C), generator=g)
-    dec = net.Decoder.__new__(net.Decoder)
-    torch.nn.Module.__init__(dec)
-    dec.K, dec.sh_dim, dec.opacity_dim, dec.scaling_dim, dec.rotation_dim = K, sh_dim, 1, 2, 4
-    dec.mlp_coarse = torch.nn.Identity()
-    opacity_shift, scaling_shift = -2.1792, -4.2
-    ref = dec.forward_coarse(feats, opacity_shift, scaling_shift)        # offset, sh, scaling, rotation, opacity
-    centers_grid = torch.rand((1, N, 3), generator=g) - 0.5
-    fake_self = types.SimpleNamespace(scene_size=1.0, n_offset_groups=16, group_centers=centers_grid)
-    ref_centers = net.Network.get_offseted_pt(fake_self, ref[0], K)
+    feats, centers_grid, K, sh_dim, opacity_shift, scaling_shift = decoder_inputs()
     mine = decoder_layout_torch(feats, centers_grid, K, sh_dim, opacity_shift, scaling_shift, 0.5 * 1.0 / 16)
-    assert torch.equal(ref_centers, mine[0])
-    for a, b in zip(ref[1:], mine[1:]):
-        assert a.shape == b.shape and torch.equal(a, b)
+    ref = Reference("decoder_layout")       # centres, sh, scaling, rotation, opacity
+    for i, t in enumerate(mine):
+        assert ref.equal(str(i), t), i
 
 
 @pytest.mark.gpu

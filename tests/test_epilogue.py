@@ -1,22 +1,21 @@
 """Fused render_img epilogue (next-row, SURVEY 8f rank 2) against the torch ops it replaces.
 
-* CPU, only where /root/reference exists: the torch restatement in lara_b200/epilogue.py is pinned
-  against the reference's own Renderer.render_img (lightning/renderer_2dgs.py) run on the CPU with
-  a stand-in rasterizer that returns fixed tensors -- the epilogue there is pure torch.
+* CPU: the torch restatement in lara_b200/epilogue.py is pinned bit for bit against what the reference's own
+  Renderer.render_img (lightning/renderer_2dgs.py) computes on the CPU with a stand-in rasterizer that returns
+  fixed tensors -- the epilogue there is pure torch (tests/golden/reference, made by
+  tests/golden/make_reference_golden.py).
 * GPU: the fused kernel vs the restatement, forward and backward (autograd), tolerance 1e-5 of the
   tensor maximum; gradients compared where alpha > 0 (the reference's D/alpha backward is NaN at
   alpha == 0, the fused one is 0)."""
-import importlib.util
-import os
 import types
 
 import numpy as np
 import pytest
 import torch
 
-from helpers import rel_err
+from helpers import Reference, rel_err
 
-REF_RENDERER = "/root/reference/lightning/renderer_2dgs.py"
+DEPTH_RATIOS = (0.0, 0.3)
 
 
 def _inputs(H, W, seed, dev="cpu"):
@@ -36,30 +35,15 @@ def _inputs(H, W, seed, dev="cpu"):
     return [t.to(dev) for t in (color, allmap, rays, vm)]
 
 
-@pytest.mark.skipif(not os.path.isfile(REF_RENDERER), reason="/root/reference not present (GPU box)")
-@pytest.mark.parametrize("depth_ratio", [0.0, 0.3])
+@pytest.mark.parametrize("depth_ratio", DEPTH_RATIOS)
 def test_torch_restatement_matches_reference_renderer_on_cpu(depth_ratio):
     from oracle.torch_restatements import render_img_epilogue_torch
-    spec = importlib.util.spec_from_file_location("ref_renderer_2dgs_epi", REF_RENDERER)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    H, W = 24, 40
-    color, allmap, rays, vm = _inputs(H, W, 0)
-
-    class FakeRasterizer:
-        def __call__(self, **kw):
-            return color, torch.zeros(kw["means3D"].shape[0], dtype=torch.int32), allmap
-    r = mod.Renderer(sh_degree=1)
-    r.set_rasterizer = lambda cam, device="cpu": FakeRasterizer()
-    cam = types.SimpleNamespace(world_view_transform=vm)
-    P = 5
-    ref = r.render_img(cam, rays, torch.zeros(P, 3), torch.zeros(P, 4, 3), torch.zeros(P, 1), torch.zeros(P, 2),
-                       torch.randn(P, 4), "cpu", depth_ratio=depth_ratio)
+    color, allmap, rays, vm = _inputs(24, 40, 0)
     mine = render_img_epilogue_torch(color, allmap, rays, vm, depth_ratio)
-    assert sorted(ref) == sorted(mine)
-    for k in ref:
-        assert ref[k].shape == mine[k].shape, k
-        assert torch.equal(ref[k], mine[k]), k
+    ref = Reference(f"epilogue_torch-{depth_ratio}")
+    assert ",".join(sorted(mine)) == ref["keys"]
+    for k in mine:
+        assert ref.equal(k, mine[k]), k
 
 
 @pytest.mark.gpu
@@ -165,16 +149,9 @@ def test_fused_activations_match_torch_activations(cuda_device, sh_degree):
     assert rel_err(a[4], b[4]) < 1e-5
 
 
-@pytest.mark.gpu
-@pytest.mark.parametrize("fused_activations", [True, False])
-def test_fast_renderer_matches_reference_pipeline(cuda_device, reference, fused_activations):
-    """lara_b200.renderer.Renderer.render_img == reference rasterizer + the torch epilogue (the
-    pipeline LaRa runs today), images and raw-parameter gradients."""
+def _pipeline_setup(dev):
     import types
     from lara_b200 import scene as S
-    from oracle.torch_restatements import render_img_epilogue_torch
-    from lara_b200.renderer import Renderer
-    dev = cuda_device
     H = W = 160
     sc = S.scene(30000, 21)
     c = S.cameras(2, H, W, 5)[1]
@@ -184,38 +161,52 @@ def test_fast_renderer_matches_reference_pipeline(cuda_device, reference, fused_
     _, _, rays, _ = _inputs(H, W, 3, dev)
     base = {"centers": sc["means3D"], "shs": sc["shs"], "opacity": torch.logit(sc["opacities"].clamp(1e-4, 1 - 1e-4)),
             "scales": torch.log(sc["scales"]), "rotations": sc["rotations"] * 0.7}
-
-    def loss_of(out):
-        mask = (out["acc_map"] > 0).detach()
-        return ((out["image"] - 0.4) ** 2).mean() + 0.2 * (out["rend_normal"] ** 2).mean() + 1000.0 * out["rend_dist"].mean() \
-            + 0.1 * (out["depth"][..., 0] * mask).mean() + out["acc_map"].mean() \
-            + 0.2 * (1 - (out["rend_normal"] * out["depth_normal"]).sum(-1)).mean()
-
-    res = []
-    # (a) this repo's fast Renderer
     raw = {k: v.to(dev).clone().requires_grad_(True) for k, v in base.items()}
-    r = Renderer(sh_degree=1, white_background=True, fused_activations=fused_activations)
-    out = r.render_img(cam, rays, raw["centers"], raw["shs"], raw["opacity"], raw["scales"], raw["rotations"], dev)
-    loss_of(out).backward()
-    res.append(({k: v.detach().cpu().numpy() for k, v in out.items()}, {k: torch.nan_to_num(v.grad).cpu().numpy() for k, v in raw.items()}))
-    # (b) reference rasterizer + torch epilogue
-    raw = {k: v.to(dev).clone().requires_grad_(True) for k, v in base.items()}
-    rs = S.settings_for(c, torch.ones(3), 1, dev, reference.GaussianRasterizationSettings)
-    img, radii, allmap = reference.GaussianRasterizer(raster_settings=rs)(
+    return c, cam, rays, raw
+
+
+def _pipeline_loss_and_outputs(out, raw):
+    mask = (out["acc_map"] > 0).detach()
+    loss = ((out["image"] - 0.4) ** 2).mean() + 0.2 * (out["rend_normal"] ** 2).mean() + 1000.0 * out["rend_dist"].mean() \
+        + 0.1 * (out["depth"][..., 0] * mask).mean() + out["acc_map"].mean() \
+        + 0.2 * (1 - (out["rend_normal"] * out["depth_normal"]).sum(-1)).mean()
+    loss.backward()
+    return {"close": {**{k: v.detach().cpu().numpy() for k, v in out.items()},
+                      **{"grad." + k: torch.nan_to_num(v.grad).cpu().numpy() for k, v in raw.items()}},
+            "scalars": {"keys": ",".join(sorted(out))}}
+
+
+def reference_pipeline_outputs(mod, dev):
+    """The pipeline LaRa runs today: the rasterizer of package `mod` + the torch epilogue."""
+    from lara_b200 import scene as S
+    from oracle.torch_restatements import render_img_epilogue_torch
+    c, cam, rays, raw = _pipeline_setup(dev)
+    rs = S.settings_for(c, torch.ones(3), 1, dev, mod.GaussianRasterizationSettings)
+    img, radii, allmap = mod.GaussianRasterizer(raster_settings=rs)(
         means3D=raw["centers"], means2D=torch.zeros_like(raw["centers"], requires_grad=True) + 0, shs=raw["shs"],
         opacities=torch.sigmoid(raw["opacity"]), scales=torch.exp(raw["scales"]),
         rotations=torch.nn.functional.normalize(raw["rotations"]), cov3D_precomp=None)
-    out = render_img_epilogue_torch(img, allmap, rays, cam.world_view_transform, 0.0)
-    loss_of(out).backward()
-    res.append(({k: v.detach().cpu().numpy() for k, v in out.items()}, {k: torch.nan_to_num(v.grad).cpu().numpy() for k, v in raw.items()}))
-    (o1, g1), (o2, g2) = res
-    assert sorted(o1) == sorted(o2) == ["acc_map", "depth", "depth_normal", "image", "rend_dist", "rend_normal"]
-    for k in o2:
-        assert o1[k].shape == o2[k].shape
-        assert rel_err(o1[k], o2[k]) < (1e-4 if k == "depth_normal" else 1e-5), k
-    for k in g1:
-        assert np.isfinite(g1[k]).all()
-        assert rel_err(g1[k], g2[k]) < 2e-4, k
+    return _pipeline_loss_and_outputs(render_img_epilogue_torch(img, allmap, rays, cam.world_view_transform, 0.0), raw)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("fused_activations", [True, False])
+def test_fast_renderer_matches_reference_pipeline(cuda_device, fused_activations):
+    """lara_b200.renderer.Renderer.render_img == reference rasterizer + the torch epilogue (the
+    pipeline LaRa runs today, stored by reference_pipeline_outputs), images and raw-parameter gradients."""
+    from lara_b200.renderer import Renderer
+    dev = cuda_device
+    _, cam, rays, raw = _pipeline_setup(dev)
+    r = Renderer(sh_degree=1, white_background=True, fused_activations=fused_activations)
+    out = r.render_img(cam, rays, raw["centers"], raw["shs"], raw["opacity"], raw["scales"], raw["rotations"], dev)
+    mine = _pipeline_loss_and_outputs(out, raw)["close"]
+    ref = Reference("fast_renderer_pipeline")
+    assert ",".join(sorted(out)) == ref["keys"] == "acc_map,depth,depth_normal,image,rend_dist,rend_normal"
+    for k in out:
+        assert ref.rel_err(k, mine[k]) < (1e-4 if k == "depth_normal" else 1e-5), k
+    for k in raw:
+        assert np.isfinite(mine["grad." + k]).all()
+        assert ref.rel_err("grad." + k, mine["grad." + k]) < 2e-4, k
 
 
 @pytest.mark.gpu

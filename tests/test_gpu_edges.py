@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import rel_err, run_candidate, to_dev
+from helpers import Reference, run_candidate, to_dev
 
 pytestmark = pytest.mark.gpu
 
@@ -47,54 +47,61 @@ def test_everything_behind_camera(cuda_device):
         assert float(np.abs(out[k]).max()) == 0.0, k
 
 
-@pytest.mark.parametrize("n_big,expect_min", [(3000, 2049), (20000, 16385), (70000, 65537)])
-def test_huge_splats_cover_every_tile(cuda_device, reference, n_big, expect_min):
-    """> 2048 instances per tile -> 1024-thread shared-memory bucket sort; > 8192 -> in-place global
-    bitonic sort; > 65536 instances in one tile is the SURVEY's stress case."""
+HUGE = [(3000, 2049), (20000, 16385), (70000, 65537)]
+PILEUP = [(2000, 16), (8000, 16), (8000, 48)]
+
+
+def huge_splats_scene(n_big):
     from lara_b200 import scene as S
-    from oracle import ref as REF
     H = W = 64
     sc = S.scene(n_big, 3)
     sc["scales"][:] = 0.6                       # every splat covers the whole image
     sc["opacities"][:] = 0.02
     sc["means3D"] *= 0.2
     sc["means3D"][::7] = sc["means3D"][0]       # exact depth ties, broken by Gaussian index
-    cam = S.cameras(1, H, W, 0)[0]
-    bg = torch.zeros(3)
-    mine = run_candidate(sc, cam, bg, cuda_device, grads=S.upstream_grads(H, W, 1))
+    return sc, S.cameras(1, H, W, 0)[0], torch.zeros(3)
+
+
+@pytest.mark.parametrize("n_big,expect_min", HUGE)
+def test_huge_splats_cover_every_tile(cuda_device, n_big, expect_min):
+    """> 2048 instances per tile -> 1024-thread shared-memory bucket sort; > 8192 -> in-place global
+    bitonic sort; > 65536 instances in one tile is the SURVEY's stress case."""
+    from lara_b200 import scene as S
+    sc, cam, bg = huge_splats_scene(n_big)
+    mine = run_candidate(sc, cam, bg, cuda_device, grads=S.upstream_grads(64, 64, 1))
     counts = mine["ranges"][:, 1] - mine["ranges"][:, 0]
     assert int(counts.max()) >= expect_min
-    scd = to_dev(sc, cuda_device)
-    st = S.settings_for(cam, bg, 1, cuda_device, reference.GaussianRasterizationSettings)
-    r = REF.forward_raw(reference, scd, st)
+    r = Reference(f"huge_splats-{n_big}")
     assert mine["num_rendered"] == r["num_rendered"]
-    assert np.array_equal(mine["point_list"], r["point_list"].cpu().numpy())
-    assert np.array_equal(mine["ranges"], r["ranges"].cpu().numpy())
-    assert np.array_equal(mine["n_contrib"][0], r["n_contrib"][0].cpu().numpy())
-    assert np.array_equal(mine["allmap"].view(np.int32), r["allmap"].cpu().numpy().view(np.int32))
+    assert r.equal("point_list", mine["point_list"])
+    assert r.equal("ranges", mine["ranges"])
+    assert r.equal("n_contrib", mine["n_contrib"][0])
+    assert r.equal("allmap", mine["allmap"])
     for k in ("g_means3D", "g_opacities", "g_scales"):
         assert np.isfinite(mine[k]).all()
 
 
-@pytest.mark.parametrize("n,H", [(2000, 16), (8000, 16), (8000, 48)])
-def test_equal_depth_pileup_is_sorted_and_not_quadratic(cuda_device, reference, n, H):
-    """Every instance of a tile has the SAME depth (the degenerate case of the depth-bucket sort: one bucket holds the
-    whole tile, ranking inside it would be quadratic -- 8192 instances = 65k steps per thread).  The sort falls back to the
-    comparison network; order (by Gaussian index, as the reference's stable sort leaves it) and a time bound are checked."""
-    from lara_b200 import rasterizer as R, scene as S
-    from oracle import ref as REF
+def pileup_scene(n, H):
+    from lara_b200 import scene as S
     sc = S.scene(n, 9)
     sc["means3D"][:] = torch.tensor([0.0, 0.0, 0.0])      # all splats at the origin: identical view-space depth
     sc["scales"][:] = 0.5
     sc["opacities"][:] = 0.01
-    cam = S.cameras(1, H, H, 0)[0]
-    bg = torch.zeros(3)
+    return sc, S.cameras(1, H, H, 0)[0], torch.zeros(3)
+
+
+@pytest.mark.parametrize("n,H", PILEUP)
+def test_equal_depth_pileup_is_sorted_and_not_quadratic(cuda_device, n, H):
+    """Every instance of a tile has the SAME depth (the degenerate case of the depth-bucket sort: one bucket holds the
+    whole tile, ranking inside it would be quadratic -- 8192 instances = 65k steps per thread).  The sort falls back to the
+    comparison network; order (by Gaussian index, as the reference's stable sort leaves it) and a time bound are checked."""
+    from lara_b200 import rasterizer as R, scene as S
+    sc, cam, bg = pileup_scene(n, H)
     mine = run_candidate(sc, cam, bg, cuda_device)
     scd = to_dev(sc, cuda_device)
-    st = S.settings_for(cam, bg, 1, cuda_device, reference.GaussianRasterizationSettings)
-    r = REF.forward_raw(reference, scd, st)
+    r = Reference(f"pileup-{n}_{H}")
     assert mine["num_rendered"] == r["num_rendered"] >= n
-    assert np.array_equal(mine["point_list"], r["point_list"].cpu().numpy())
+    assert r.equal("point_list", mine["point_list"])
     assert len(np.unique(mine["depths"][mine["radii"] > 0].view(np.int32))) == 1
     # time: the whole forward of this tiny image, repeated; a quadratic rank loop takes milliseconds per tile
     stm = S.settings_for(cam, bg, 1, cuda_device, R.GaussianRasterizationSettings)
@@ -128,22 +135,23 @@ def test_sorted_by_depth_then_index_within_each_tile(cuda_device):
     assert total == out["num_rendered"] == int(out["tiles_touched"].sum())
 
 
-def test_opacity_extremes_and_saturation(cuda_device, reference):
+def opacity_extremes_scene():
     from lara_b200 import scene as S
-    from oracle import ref as REF
     sc = S.scene(8000, 6)
     sc["opacities"][0::3] = 1.0        # alpha clamps at 0.99, pixels saturate (early termination)
     sc["opacities"][1::3] = 1e-5       # never reaches 1/255
     sc["scales"] *= 3.0
-    cam = S.cameras(1, 128, 128, 0)[0]
-    bg = torch.full((3,), 0.5)
+    return sc, S.cameras(1, 128, 128, 0)[0], torch.full((3,), 0.5)
+
+
+def test_opacity_extremes_and_saturation(cuda_device):
+    from lara_b200 import scene as S
+    sc, cam, bg = opacity_extremes_scene()
     gc, ga = S.upstream_grads(128, 128, 2)
     mine = run_candidate(sc, cam, bg, cuda_device, grads=(gc, ga))
-    scd = to_dev(sc, cuda_device)
-    st = S.settings_for(cam, bg, 1, cuda_device, reference.GaussianRasterizationSettings)
-    r = REF.forward_raw(reference, scd, st)
-    assert np.array_equal(mine["n_contrib"][0], r["n_contrib"][0].cpu().numpy())
-    assert np.array_equal(mine["allmap"].view(np.int32), r["allmap"].cpu().numpy().view(np.int32))
+    r = Reference("opacity_extremes")
+    assert r.equal("n_contrib", mine["n_contrib"][0])
+    assert r.equal("allmap", mine["allmap"])
     assert float(mine["accum"][0].min()) < 1e-3           # saturated pixels exist
     assert float(np.abs(mine["g_opacities"][1::3]).max()) == 0.0
     for k in ("g_means3D", "g_sh", "g_opacities", "g_scales", "g_rotations"):
@@ -164,42 +172,49 @@ def test_capacity_overflow_reruns_binning(cuda_device, monkeypatch):
     assert np.array_equal(small["allmap"].view(np.int32), base["allmap"].view(np.int32))
 
 
-def test_colors_precomp_path(cuda_device, reference):
+def colors_precomp_outputs(mod, dev):
+    """Colour and aux maps (bit for bit) and the gradients of colors_precomp and means3D through package `mod`."""
     from lara_b200 import scene as S
-    import diff_surfel_rasterization as DSR
     sc = S.scene(5000, 8)
     cam = S.cameras(1, 128, 128, 0)[0]
-    bg = torch.ones(3)
-    scd = to_dev(sc, cuda_device)
-    colors = torch.rand(5000, 3, device=cuda_device)
-    gc, ga = [t.to(cuda_device) for t in S.upstream_grads(128, 128, 0)]
-    res = []
-    for mod in (DSR, reference):
-        st = S.settings_for(cam, bg, 1, cuda_device, mod.GaussianRasterizationSettings)
-        c_in = colors.clone().requires_grad_(True)
-        m3 = scd["means3D"].clone().requires_grad_(True)
-        rast = mod.GaussianRasterizer(raster_settings=st)
-        c, rd, am = rast(means3D=m3, means2D=torch.zeros_like(m3), colors_precomp=c_in, opacities=scd["opacities"],
-                         scales=scd["scales"], rotations=scd["rotations"])
-        torch.autograd.backward((c, am), (gc, ga))
-        res.append((c.detach().cpu().numpy(), am.detach().cpu().numpy(), c_in.grad.cpu().numpy(), m3.grad.cpu().numpy()))
-    assert np.array_equal(res[0][0].view(np.int32), res[1][0].view(np.int32))     # no SH -> colour bit-exact too
-    assert np.array_equal(res[0][1].view(np.int32), res[1][1].view(np.int32))
-    assert rel_err(res[0][2], res[1][2]) < 1e-4 and rel_err(res[0][3], res[1][3]) < 1e-4
+    scd = to_dev(sc, dev)
+    colors = torch.rand((5000, 3), generator=torch.Generator().manual_seed(8)).to(dev)
+    gc, ga = [t.to(dev) for t in S.upstream_grads(128, 128, 0)]
+    st = S.settings_for(cam, torch.ones(3), 1, dev, mod.GaussianRasterizationSettings)
+    c_in = colors.clone().requires_grad_(True)
+    m3 = scd["means3D"].clone().requires_grad_(True)
+    c, rd, am = mod.GaussianRasterizer(raster_settings=st)(
+        means3D=m3, means2D=torch.zeros_like(m3), colors_precomp=c_in, opacities=scd["opacities"],
+        scales=scd["scales"], rotations=scd["rotations"])
+    torch.autograd.backward((c, am), (gc, ga))
+    return {"exact": {"color": c.detach().cpu().numpy(), "allmap": am.detach().cpu().numpy()},
+            "close": {"g_colors": c_in.grad.cpu().numpy(), "g_means3D": m3.grad.cpu().numpy()}}
 
 
-def test_mark_visible_matches_reference(cuda_device, reference):
+def test_colors_precomp_path(cuda_device):
+    import diff_surfel_rasterization as DSR
+    mine = colors_precomp_outputs(DSR, cuda_device)
+    r = Reference("colors_precomp")
+    assert r.equal("color", mine["exact"]["color"])     # no SH -> colour bit-exact too
+    assert r.equal("allmap", mine["exact"]["allmap"])
+    for k, v in mine["close"].items():
+        assert r.rel_err(k, v) < 1e-4, k
+
+
+def mark_visible_scene():
+    from lara_b200 import scene as S
+    sc = S.scene(10000, 9)
+    sc["means3D"] = sc["means3D"] * 4.0          # some points end up behind the near plane
+    return sc, S.cameras(1, 64, 64, 0)[0]
+
+
+def test_mark_visible_matches_reference(cuda_device):
     from lara_b200 import scene as S
     import diff_surfel_rasterization as DSR
-    sc = S.scene(10000, 9)
-    cam = S.cameras(1, 64, 64, 0)[0]
-    sc["means3D"] = sc["means3D"] * 4.0          # some points end up behind the near plane
-    pts = sc["means3D"].to(cuda_device)
-    outs = []
-    for mod in (DSR, reference):
-        st = S.settings_for(cam, torch.ones(3), 1, cuda_device, mod.GaussianRasterizationSettings)
-        outs.append(mod.GaussianRasterizer(raster_settings=st).markVisible(pts).cpu().numpy())
-    assert outs[0].dtype == np.bool_ and np.array_equal(outs[0], outs[1]) and 0 < outs[0].sum() < 10000
+    sc, cam = mark_visible_scene()
+    st = S.settings_for(cam, torch.ones(3), 1, cuda_device, DSR.GaussianRasterizationSettings)
+    vis = DSR.GaussianRasterizer(raster_settings=st).markVisible(sc["means3D"].to(cuda_device)).cpu().numpy()
+    assert vis.dtype == np.bool_ and Reference("mark_visible").equal("visible", vis) and 0 < vis.sum() < 10000
 
 
 def test_non_contiguous_inputs_and_debug_flag(cuda_device):

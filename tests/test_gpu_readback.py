@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import to_dev
+from helpers import Reference, to_dev
 
 pytestmark = pytest.mark.gpu
 
@@ -25,10 +25,9 @@ def _render(DSR, leaves, st):
                 scales=leaves["scales"], rotations=leaves["rotations"])
 
 
-def test_ctx_num_rendered_is_lazy_and_correct(cuda_device, reference):
+def test_ctx_num_rendered_is_lazy_and_correct(cuda_device):
     import diff_surfel_rasterization as DSR
     from lara_b200 import rasterizer as R, scene as S
-    from oracle import ref as REF
     sc = S.scene(20000, 11)
     scd = to_dev(sc, cuda_device)
     cam = S.cameras(1, 256, 256, 1)[0]
@@ -36,8 +35,7 @@ def test_ctx_num_rendered_is_lazy_and_correct(cuda_device, reference):
     color, radii, allmap = _render(DSR, _leaves(scd), st)
     n = color.grad_fn.num_rendered                     # the reference stores an int on ctx (DSR __init__.py:95)
     assert isinstance(n, (int, R.LazyCount))
-    ref_st = S.settings_for(cam, torch.ones(3), 1, cuda_device, reference.GaussianRasterizationSettings)
-    assert int(n) == REF.forward_raw(reference, scd, ref_st)["num_rendered"]
+    assert int(n) == Reference("ctx_num_rendered")["num_rendered"]      # what the reference's forward counts
     assert n == int(n) and f"{n}" == str(int(n))
 
 

@@ -1,23 +1,20 @@
 """Fused loss -> dL/d(render_img outputs) producer (next-row, SURVEY 8f rank 3).
 
-* CPU, only where /root/reference exists: the torch restatement (oracle/torch_restatements.lara_loss_torch) is
-  pinned bit-exactly against the reference's own ``Losses.forward`` (lightning/loss.py) with ``pytorch_msssim``
-  (absent here) replaced by a stub whose MS_SSIM returns 1 -- the MSE / distortion / normal-consistency terms and
-  their autograd gradients are the reference's.
+* CPU: the torch restatement (oracle/torch_restatements.lara_loss_torch) is pinned bit-exactly against what the
+  reference's own ``Losses.forward`` (lightning/loss.py) computes with ``pytorch_msssim`` replaced by a stub whose
+  MS_SSIM returns 1 -- the MSE / distortion / normal-consistency terms and their autograd gradients are the
+  reference's (tests/golden/reference, made by tests/golden/make_reference_golden.py).
 * GPU: ``lara_b200.loss.scene_loss`` (two CUDA kernels on the stacked planar buffers) vs the restatement on the
   concatenated [H, V*W, C] layout, loss terms and all four gradient maps, and end to end through
   ``render_scene_views`` to the Gaussian-parameter gradients."""
-import importlib.util
-import os
-import sys
 import types
 
 import pytest
 import torch
 
-from helpers import rel_err
+from helpers import Reference, rel_err
 
-REF_LOSS = "/root/reference/lightning/loss.py"
+ITERATIONS = (10, 5000)
 
 
 def _fake_outputs(B, V, H, W, seed, dev="cpu"):
@@ -32,44 +29,21 @@ def _fake_outputs(B, V, H, W, seed, dev="cpu"):
     return {k: v.to(dev) for k, v in out.items()}, tar.to(dev)
 
 
-@pytest.mark.skipif(not os.path.isfile(REF_LOSS), reason="/root/reference not present (GPU box)")
-@pytest.mark.parametrize("it", [10, 5000])
+@pytest.mark.parametrize("it", ITERATIONS)
 def test_loss_restatement_matches_reference_losses_on_cpu(it):
     from oracle.torch_restatements import lara_loss_torch
-    stub = types.ModuleType("pytorch_msssim")
-
-    class MS_SSIM(torch.nn.Module):          # stand-in: constant 1 -> contributes 0.5 * (1 - 1) = 0
-        def __init__(self, **kw):
-            super().__init__()
-
-        def forward(self, a, b):
-            return torch.ones((), dtype=a.dtype)
-    stub.MS_SSIM = MS_SSIM
-    saved = sys.modules.get("pytorch_msssim")
-    sys.modules["pytorch_msssim"] = stub
-    try:
-        spec = importlib.util.spec_from_file_location("ref_lara_loss", REF_LOSS)
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-    finally:
-        if saved is None:
-            sys.modules.pop("pytorch_msssim", None)
-        else:
-            sys.modules["pytorch_msssim"] = saved
     out, tar = _fake_outputs(2, 3, 16, 24, 0)
-    la = {k: v.clone().requires_grad_(k != "acc_map") for k, v in out.items()}
     lb = {k: v.clone().requires_grad_(k != "acc_map") for k, v in out.items()}
-    ref_loss, ref_stats = mod.Losses()({"tar_rgb": tar}, la, it)
     my_loss, my_stats = lara_loss_torch(lb, tar, it)
-    assert torch.equal(ref_loss.reshape(()), my_loss.reshape(()))
+    ref = Reference(f"loss-{it}")
+    assert ref.equal("loss", my_loss.reshape(()))
     for k in my_stats:
-        assert torch.equal(ref_stats[k].reshape(-1), my_stats[k].reshape(-1)), k
-    ref_loss.backward(); my_loss.backward()
-    for k in la:
-        if la[k].grad is None:
-            assert lb[k].grad is None, k
-        else:
-            assert torch.equal(la[k].grad, lb[k].grad), k
+        assert ref.equal("stat." + k, my_stats[k].reshape(-1)), k
+    my_loss.backward()
+    assert ",".join(sorted(k for k, v in lb.items() if v.grad is None)) == ref["no_grad"]
+    for k in lb:
+        if lb[k].grad is not None:
+            assert ref.equal("grad." + k, lb[k].grad), k
 
 
 @pytest.mark.gpu
